@@ -24,6 +24,15 @@ the 40-byte shard aggregate plus the 32-byte output checksum hopping rank to ran
 (mtz_dev_finish_exchange).  Rank 0 then measures, in one process over all N GPUs, `e2e` and the
 fan-out of the processed stream to P attached peers (BASELINE configs[3]/[4]).
 
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned as DIR/<name>.npy
+(float32 / float64, u64 values as exact (hi32, lo32) pairs): per chunk j the output stream's size
+(chunkj_output_bytes), the running checksums the finish call returned (chunkj_carry, chunkj_carry_out)
+and 128 / (number of chunks) windows of 64 KiB of the output stream at seeded offsets
+(chunkj_output_sample, chunkj_output_sample_offsets), plus the END checksum (end_checksum); with
+`--workload verify` the step's size, carries and END checksum; with `--impl reference` what the oracle
+returned for its bounded sample, under the same names without the chunk prefix.  The inputs
+are seeded, so two builds run with the same arguments can be compared array for array.
+
 `--workload verify` keeps round 1's headline (configs[1]: 16 GiB uncompressed, Fletcher-4 only) as a
 selectable workload; the default run reports it as `workloads.verify`.
 """
@@ -62,7 +71,13 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-reencode", action="store_true", help="skip the certificate-off resident leg (N=1)")
     ap.add_argument("--recsize", type=int, default=131072, help="DRR_WRITE logical size (dataset recordsize)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy "
+                         "(see the module docstring), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 class ClockSampler(object):
@@ -217,6 +232,43 @@ def verify_config(gib_per_gpu):
             "metric_bytes": "input stream bytes"}
 
 
+# ------------------------------------------------------------------------------ output dump --
+DUMP_WINDOW = 65536          # bytes per sampled window of an output stream
+DUMP_SAMPLE_BYTES = 8 << 20  # sampled output bytes over all chunks: 32 MiB as float32
+
+
+def u64_words(vals):
+    """u64 values as float64 (hi32, lo32) pairs: exact, unlike a u64 -> float64 cast"""
+    import numpy as np
+    v = np.asarray(vals, dtype=np.uint64).reshape(-1)
+    return np.stack([v >> np.uint64(32), v & np.uint64(0xffffffff)], axis=1).astype(np.float64)
+
+
+def output_sample(d_out, out_bytes, in_bytes, seed, windows):
+    """`windows` windows of DUMP_WINDOW bytes of the device output stream d_out[:out_bytes] at
+    offsets drawn with `seed` over the INPUT size, which is identical between builds -> (bytes as
+    float32, -1 past the end of the output; window offsets as float64)"""
+    import numpy as np
+    import torch
+    rng = np.random.default_rng(seed)
+    offs = np.sort(rng.integers(0, max(1, in_bytes - DUMP_WINDOW + 1), size=windows))
+    idx = (torch.from_numpy(offs).to(d_out.device)[:, None] +
+           torch.arange(DUMP_WINDOW, device=d_out.device)[None, :]).reshape(-1)
+    vals = d_out[idx.clamp(max=max(0, out_bytes - 1))].float()
+    vals[idx >= out_bytes] = -1.0
+    return vals.cpu().numpy(), offs.astype(np.float64)
+
+
+def dump_outputs(dirname, arrays):
+    """DIR/<name>.npy for every array, float32 / float64 only"""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- reference arm --
 def run_reference(args):
     """CPU arm: the oracle port of the path's arithmetic on all host threads, each step a bounded
@@ -243,6 +295,8 @@ def run_reference(args):
             rc, secs, st = O.mt_verify(s, nthreads)
             assert rc == 0
             t.append(secs)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"end_checksum": u64_words(st.end_cksum.tuple())})
         ms = 1e3 * sum(t) / len(t)
         val = s.size / GIB / (ms / 1e3)
         cfg = verify_config(gib)
@@ -260,6 +314,12 @@ def run_reference(args):
         for _ in range(args.steps):
             n, secs = cpu_recompress(O, src, out, nthreads)
             t.append(secs)
+        if args.dump_outputs:
+            import torch
+            smp, offs = output_sample(torch.from_numpy(out), n, src.size, seed=0x4d545a,
+                                      windows=DUMP_SAMPLE_BYTES // DUMP_WINDOW)
+            dump_outputs(args.dump_outputs, {"output_sample": smp, "output_sample_offsets": offs,
+                                             "output_bytes": np.array([n], dtype=np.float64)})
         ms = 1e3 * sum(t) / len(t)
         val = src.size / GIB / (ms / 1e3)
         cfg = recompress_config(gib)
@@ -440,13 +500,18 @@ def run_verify_resident(args, O, local, steps, warm, peak):
         torch.cuda.synchronize()
         e0.record(st)
         for _ in range(steps):
-            step()
+            fin = step()
         e1.record(st)
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / steps
         s1 = g.stats()
         k1_ms = (s1["k1_ms"] - s0["k1_ms"]) / max(1, s1["k1_launches"] - s0["k1_launches"])
         end_ck = g.end_checksum()
+        if args.dump_outputs and args.workload == "verify":
+            # VERIFY hands the input on unchanged: what a step returns is its verdict
+            dump_outputs(args.dump_outputs, {"output_bytes": np.array([fin[0]], dtype=np.float64),
+                                             "carry": u64_words(fin[1]), "carry_out": u64_words(fin[2]),
+                                             "end_checksum": u64_words(end_ck)})
         res.update({"value": round(s.size / GIB / (ms / 1e3), 3), "unit": "GiB/s", "ms_per_step": round(ms, 4),
                     "steps": steps, "gpu_launches": int((s1["kernel_launches"] - s0["kernel_launches"]) // steps),
                     "config": verify_config(gib),
@@ -592,6 +657,7 @@ def run_ours(args):
     acc = {"k3_ms": 0.0, "codec_ms": 0.0, "k3_launches": 0.0, "kernel_launches": 0.0,
            "lz4_certified": 0.0, "lz4_encoded": 0.0}
     end_ck = [None]
+    finished = [None] * CH                 # (out_bytes, carry, carry_out) of each chunk, last step
 
     def submit(k):
         c, g, st_ = chunks[k], hs[k % len(hs)], sts[k % len(hs)]
@@ -608,9 +674,12 @@ def run_ours(args):
         for k in range(CH):
             g = hs[k % len(hs)]
             if world == 1:
-                ob, _, _ = g.dev_finish()
+                fin = g.dev_finish()
             else:
-                ob, _, _, base = g.dev_finish_exchange(round_base=base, flags=chunks[k]["flags"])
+                fin = g.dev_finish_exchange(round_base=base, flags=chunks[k]["flags"])
+                base = fin[3]
+            finished[k] = fin[:3]
+            ob = fin[0]
             obs.append(ob)
             s_ = g.stats()                     # dev_reset() zeroes the counters per chunk
             for key in acc:
@@ -659,6 +728,20 @@ def run_ours(args):
     value = total_bytes / GIB / (ms_step / 1e3)
     k3_ms, codec_ms, k3_launches, launches, n_cert, n_enc = [float(x) for x in ksum.tolist()]
     end_ck = end_ck[0]
+    if args.dump_outputs:
+        # the last timed step's output stream of every chunk this rank finished (N = 1: the whole
+        # stream), sampled, and the checksums and sizes the finish calls returned
+        arrays = {}
+        for c, (ob, carry, carry_out) in zip(chunks, finished):
+            tag = "chunk%d_" % c["j"]
+            arrays[tag + "output_sample"], arrays[tag + "output_sample_offsets"] = output_sample(
+                c["d_out"], ob, c["bytes"], seed=0x4d545a + c["j"],
+                windows=max(1, DUMP_SAMPLE_BYTES // DUMP_WINDOW // C_ALL))
+            arrays[tag + "output_bytes"] = np.array([ob], dtype=np.float64)
+            arrays[tag + "carry"], arrays[tag + "carry_out"] = u64_words(carry), u64_words(carry_out)
+        if end_ck is not None:
+            arrays["end_checksum"] = u64_words(end_ck)
+        dump_outputs(args.dump_outputs, arrays)
     # the same resident step with the certificate switched off (MTZ_FLAG_REENCODE_ALL): every record
     # goes through the serial matcher -- what RECOMPRESS costs on a stream made by ANOTHER encoder
     reenc = None

@@ -1,5 +1,5 @@
 """CPU: the parts of bench.py that do not need a GPU -- argument defaults, the CPU-baseline
-object, the clock sampler's degraded path and the reference arm's JSON line."""
+object, the clock sampler's degraded path and the reference arm's JSON line and output dump."""
 import json
 import os
 import subprocess
@@ -32,10 +32,11 @@ def test_defaults_and_cpu_baseline_object(oracle):
     assert c["sm_mhz"] is None and c["reasons"]
 
 
-def test_reference_arm_prints_the_contract_line():
+def test_reference_arm_prints_the_contract_line(tmp_path):
+    dump = str(tmp_path / "outputs")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                        "--warmup", "1", "--ref-gib", "0.25"], stdout=subprocess.PIPE, stderr=subprocess.PIPE,
-                       text=True, timeout=280, cwd=ROOT)
+                        "--warmup", "1", "--ref-gib", "0.25", "--dump-outputs", dump], stdout=subprocess.PIPE,
+                       stderr=subprocess.PIPE, text=True, timeout=280, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     d = json.loads(r.stdout.strip().splitlines()[-1])
     for k in ("impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
@@ -45,6 +46,15 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert "workload" in d["config"] and d["gpu_launches"] == 0
+    # --dump-outputs: the last step's output stream, sampled, as float arrays of at most 64 MB in all
+    import numpy as np
+    out = {f[:-4]: np.load(os.path.join(dump, f)) for f in os.listdir(dump)}
+    assert sorted(out) == ["output_bytes", "output_sample", "output_sample_offsets"]
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    smp, n = out["output_sample"], int(out["output_bytes"][0])
+    assert n > 0 and smp.size == out["output_sample_offsets"].size * 65536
+    assert smp.min() >= 0 and smp.max() <= 255 and np.all(smp == np.round(smp))
 
 
 def test_restated_plumbing_pump_pair_moves_the_stream_unchanged():
